@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            (N > 1: launched under torch.distributed.run)
     python bench.py --impl reference --steps K --warmup W    (reference arm: the UNMODIFIED reference on the host cores)
     python bench.py --config c2|c3|c5  --mode native|dropin  --precision tf32|3xtf32   (other BASELINE.json configs / modes)
+    python bench.py ... --dump-outputs DIR   (also write what the last timed step computed as DIR/<name>.npy)
 
 One "step" (default config c3, BASELINE.json configs[2]; configs[3] when N > 1) = one full GAN step: 2 discriminator updates + 1
 generator update, hinge + grid-cell losses, Adam, on a synthetic batch of 16 4->18-frame 256x256 radar sequences per GPU (weak
@@ -276,6 +277,32 @@ def emit(line: dict):
         os.write(_REAL_STDOUT, data)
 
 
+DUMP_MAX_ELEMS = 8 << 20      # per output array (32 MB of fp32); a larger one is written as a fixed, seeded sample of this many elements
+DUMP_PARAM_SAMPLE = 1 << 20   # elements sampled from each network's updated parameters
+
+
+def _seeded_sample(t, k):
+    idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:k].sort().values
+    return t.reshape(-1)[idx.to(t.device)]
+
+
+def dump_outputs(path, outputs, nets=None):
+    """Write the arrays the last timed step returned (`outputs`: name -> tensor) as path/<name>.npy in float32, and for a training step
+    `nets` = (generator, discriminator): a fixed, seeded sample of each network's parameters after that step's update, flattened in
+    `.parameters()` order.  Arrays over DUMP_MAX_ELEMS elements are flattened and sampled the same way; at most ~40 MB in all."""
+    import numpy as np
+
+    arrays = {k: v.detach() for k, v in outputs.items()}
+    for name, net in zip(("generator_params", "discriminator_params"), nets or ()):
+        flat = torch.cat([p.detach().reshape(-1) for p in net.parameters()])
+        arrays[name] = _seeded_sample(flat, min(DUMP_PARAM_SAMPLE, flat.numel()))
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        if t.numel() > DUMP_MAX_ELEMS:
+            t = _seeded_sample(t, DUMP_MAX_ELEMS)
+        np.save(os.path.join(path, name + ".npy"), t.float().cpu().numpy())
+
+
 def main():
     # stdout must carry exactly one JSON line, but libraries print there too (NCCL's "NCCL version ..." banner under torchrun):
     # point fd 1 at stderr for the duration of the run and keep the real stdout for emit()
@@ -301,7 +328,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-ref-gpu", action="store_true", help="skip the reference's own GPU path (reference_gpu_eager)")
     ap.add_argument("--cpu-batch", type=int, default=1)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (and, for training, a fixed sample of the "
+                         "updated parameters) as DIR/<name>.npy, to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     c = CONFIGS[args.config]
     args.batch = args.batch or c["batch"]
     args.generation_steps = args.generation_steps or c["k"]
@@ -403,8 +435,11 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
+    last = {}
+
     def step_resident():
-        return run_step(x, y)
+        last["out"] = run_step(x, y)
+        return last["out"]
 
     def step_e2e():
         xi = host_x.to(dev, non_blocking=True)
@@ -439,6 +474,8 @@ def main():
         sampler.start()
     ms, launches = timed(step_resident, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last["out"], None if inference else (gen, disc))
     step_e2e()
     ms_e2e, _ = timed(step_e2e, args.steps)
 

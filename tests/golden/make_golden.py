@@ -1,16 +1,22 @@
-"""Generate golden fixtures by running the UNMODIFIED reference (/root/reference) on CPU.
+"""Generate golden fixtures by running the UNMODIFIED reference (openclimatefix/skillful_nowcasting) on CPU:
 
-Run in the build container only (the GPU box has no /root/reference):
+    DGMR_REFERENCE=<checkout of the reference> python tests/golden/make_golden.py
 
-    python tests/golden/make_golden.py
-
-Writes tests/golden/c1_gan.pt.  The reference has no golden vectors of its own for the hot
-path (SURVEY.md 8c), so these fixtures — outputs of the reference itself on seeded inputs —
-are what pins the oracle (tests/test_oracle.py) and, through it, the CUDA path.
+Writes, under tests/golden/:
+  c1_gan.pt                      BASELINE config C1 through the reference's generator, discriminators and losses (eval and
+                                 train): outputs, losses, gradient summaries, mutated buffers, and a digest of every tensor of
+                                 the seeded construction
+  reference_blocks.pt            each building block of the reference on small seeded inputs (tests/test_oracle.py)
+  reference_wrapper_losses.json  the losses the reference's own `DGMR.training_step` logs (tests/test_host_logic.py)
+The reference has no golden vectors of its own for the hot path (SURVEY.md 8c), so these fixtures — outputs of the reference
+itself on seeded inputs — are what pins the oracle and, through it, the CUDA path; the tests need no copy of the reference.
+The C1 generator outputs and the buffers of more than 1024 elements are stored as a fixed random sample of their elements plus
+whole-tensor statistics (sample_tensor; parity_util.rel_err compares against that form), which keeps every file below 1 MB.
 
 Import bypass (SURVEY.md 8c): `import dgmr` fails because dgmr/__init__.py pulls in
 pytorch_lightning; registering a bare package object lets the hot-path sub-modules import.
 """
+import json
 import os
 import sys
 import types
@@ -18,7 +24,10 @@ import types
 import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = os.environ.get("DGMR_REFERENCE", "/root/reference")
+sys.path[:0] = [os.path.dirname(HERE), os.path.dirname(os.path.dirname(HERE))]
+from parity_util import tensor_digest  # noqa: E402
+
+REF = os.environ.get("DGMR_REFERENCE", "")
 
 
 def import_reference():
@@ -62,17 +71,42 @@ def state_checksum(sd):
 
 
 def summarize_grads(named):
-    """Full tensors are too big to commit (G 13 M / D 45 M params): keep exact small ones,
-    and (sum, L2 norm, first 64 values) of the rest."""
+    """Full tensors are too big to commit (G 13 M / D 45 M params): (sum, L2 norm, first 64 values) of each, what
+    parity_util.compare_grads compares."""
+    return {k: {"sum": float(g.detach().double().sum()), "norm": float(g.detach().double().norm()),
+                "head": g.detach().flatten()[:64].clone()} for k, g in named.items()}
+
+
+def sample_tensor(t, k, seed=0):
+    """A fixed random subset of k of t's elements (flat indices and values) with t's max |.|, L2 norm and sum (fp64)."""
+    t = t.detach().flatten()
+    idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(seed))[:k].sort().values
+    return {"numel": t.numel(), "idx": idx.int(), "val": t[idx].clone(), "absmax": float(t.double().abs().max()),
+            "norm": float(t.double().norm()), "sum": float(t.double().sum())}
+
+
+def construction_record(sd):
+    """Per tensor of a freshly constructed state dict: its digest, except for the spectral-norm vectors u, v.  Those come out of
+    power iterations at construction, whose float rounding depends on the host's BLAS and thread count; they get a 32-element
+    sample_tensor (as plain lists) instead."""
     out = {}
-    for k, g in named.items():
-        g = g.detach()
-        ent = {"sum": float(g.double().sum()), "norm": float(g.double().norm()),
-               "head": g.flatten()[:64].clone()}
-        if g.numel() <= 4096:
-            ent["full"] = g.clone()
-        out[k] = ent
+    for k, v in sd.items():
+        if k.endswith("._u") or k.endswith("._v"):
+            s = sample_tensor(v, 32)
+            out[k] = dict(s, idx=s["idx"].tolist(), val=s["val"].tolist())
+        else:
+            out[k] = tensor_digest(v)
     return out
+
+
+def shrink(res, out_k=8192, state_max=1024, state_k=256):
+    """Sample the generator outputs and the large buffers (spectral-norm v vectors) of a run_case result in place."""
+    res["out"] = sample_tensor(res["out"], out_k)
+    for key in ("g_state_after", "d_state_after"):
+        for k, v in res.get(key, {}).items():
+            if v.numel() > state_max:
+                res[key][k] = sample_tensor(v, state_k)
+    return res
 
 
 def build_reference_gan(cfg, seed=0):
@@ -142,7 +176,70 @@ def run_case(gen, disc, g0, d0, x, y, training, seed):
     return res
 
 
+def block_record():
+    """Each building block of the reference on seeded inputs, in train then eval mode (train mode moves the spectral-norm vectors and
+    BatchNorm statistics the eval forward then uses): the initial state, and the output and the state after each forward."""
+    import_reference()
+    from dgmr.common import DBlock, GBlock, LBlock, UpsampleGBlock
+    from dgmr.layers import AttentionLayer, ConvGRU
+
+    sd = lambda m: {k: v.clone() for k, v in m.state_dict().items()}  # noqa: E731
+    torch.manual_seed(3)
+    cases = [
+        ("g_block", GBlock(16, 16), torch.rand(2, 16, 8, 8)),
+        ("upsample_g_block", UpsampleGBlock(16, 8), torch.rand(2, 16, 8, 8)),
+        ("d_block", DBlock(8, 16), torch.rand(2, 8, 8, 8)),
+        ("d_block_3d", DBlock(4, 8, conv_type="3d", first_relu=False), torch.rand(2, 4, 6, 8, 8)),
+        ("d_block_keep_same_output", DBlock(8, 8, keep_same_output=True), torch.rand(2, 8, 4, 4)),
+        ("l_block", LBlock(8, 24), torch.rand(1, 8, 4, 4)),
+    ]
+    blocks = []
+    for name, mod, x in cases:
+        rec = {"name": name, "x": x, "state": sd(mod)}     # the eval forward starts from rec["train"]["state_after"]
+        for tr in (True, False):
+            mod.train(tr)
+            with torch.no_grad():
+                out = mod(x)
+            rec["train" if tr else "eval"] = {"out": out, "state_after": sd(mod)}
+        blocks.append(rec)
+    att = AttentionLayer(48, 48)
+    with torch.no_grad():
+        att.gamma.fill_(0.7)
+    x = torch.randn(1, 48, 4, 4)
+    with torch.no_grad():
+        attention = {"state": sd(att), "x": x, "out": att(x)}
+    gru = ConvGRU(24 + 8, 8)
+    xs, h = [torch.rand(2, 24, 8, 8) for _ in range(3)], torch.rand(2, 8, 8, 8)
+    state = sd(gru)
+    with torch.no_grad():
+        conv_gru = {"state": state, "xs": xs, "h": h, "out": gru(xs, h)}
+    return {"blocks": blocks, "attention": attention, "conv_gru": conv_gru}
+
+
+WRAPPER_CFG = dict(forecast_steps=2, output_shape=128, latent_channels=288, context_channels=48)
+
+
+def wrapper_losses():
+    """The losses the reference's own DGMR.training_step logs for one step on seeded inputs (reference modules, stubbed Lightning:
+    baseline/reference_arm.py), for generation_steps 1 and 2."""
+    from baseline import reference_arm as R
+
+    os.environ["DGMR_REFERENCE"] = REF
+    torch.manual_seed(1)
+    x, y = torch.rand(2, 4, 1, 128, 128), torch.rand(2, 2, 1, 128, 128)
+    out = {"cfg": WRAPPER_CFG, "init_seed": 0, "data_seed": 1, "step_seed": 2}
+    for k in (1, 2):
+        model = R.build_dgmr(WRAPPER_CFG, generation_steps=k, dropin=False, anomaly=False, seed=0)
+        torch.manual_seed(2)
+        out[f"generation_steps={k}"] = {name: float(v) for name, v in R.training_step_fn(model, x, y)().items()}
+    for name in [name for name in sys.modules if name == "dgmr" or name.startswith("dgmr.")]:
+        del sys.modules[name]
+    return out
+
+
 def main():
+    if not os.path.isfile(os.path.join(REF, "dgmr", "dgmr.py")):
+        sys.exit("set DGMR_REFERENCE to a checkout of openclimatefix/skillful_nowcasting")
     cfg = C1
     gen, disc = build_reference_gan(cfg, seed=0)
     with torch.no_grad():
@@ -154,9 +251,10 @@ def main():
     x = torch.rand(b, 4, 1, s, s)
     y = torch.rand(b, t, 1, s, s)
     fix = {"cfg": cfg, "g_checksum": state_checksum(g0), "d_checksum": state_checksum(d0),
+           "g_digest": construction_record(g0), "d_digest": construction_record(d0),
            "init_seed": 0, "data_seed": 1, "seed": 2, "gamma": 0.5, "torch_version": str(torch.__version__)}
-    fix["eval"] = run_case(gen, disc, g0, d0, x, y, False, 2)
-    fix["train"] = run_case(gen, disc, g0, d0, x, y, True, 2)
+    fix["eval"] = shrink(run_case(gen, disc, g0, d0, x, y, False, 2))
+    fix["train"] = shrink(run_case(gen, disc, g0, d0, x, y, True, 2))
     # RNG draws the reference makes inside that forward, recorded for documentation
     torch.manual_seed(2)
     fix["z"] = torch.normal(torch.zeros(8, s // 32, s // 32, 1), torch.ones(8, s // 32, s // 32, 1))
@@ -164,8 +262,16 @@ def main():
     path = os.path.join(HERE, "c1_gan.pt")
     torch.save(fix, path)
     print("wrote", path, os.path.getsize(path) / 1e6, "MB")
-    print("eval out sum", float(fix["eval"]["out"].double().sum()), "scores", fix["eval"]["scores"].flatten().tolist())
-    print("train out sum", float(fix["train"]["out"].double().sum()), "d_loss", float(fix["train"]["d_loss"]))
+    print("eval out sum", fix["eval"]["out"]["sum"], "scores", fix["eval"]["scores"].flatten().tolist())
+    print("train out sum", fix["train"]["out"]["sum"], "d_loss", float(fix["train"]["d_loss"]))
+    path = os.path.join(HERE, "reference_blocks.pt")
+    torch.save(block_record(), path)
+    print("wrote", path, os.path.getsize(path) / 1e6, "MB")
+    path = os.path.join(HERE, "reference_wrapper_losses.json")
+    with open(path, "w") as f:
+        json.dump(wrapper_losses(), f, indent=1)
+        f.write("\n")
+    print("wrote", path)
 
 
 if __name__ == "__main__":

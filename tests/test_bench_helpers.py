@@ -40,6 +40,29 @@ def test_reference_arm_other_ranks_exit_silently():
     assert r.returncode == 0 and r.stdout.strip() == ""
 
 
+def test_dump_outputs_writes_float32_and_a_fixed_sample_of_large_arrays(tmp_path, monkeypatch):
+    """--dump-outputs: one float32 .npy per returned array, parameter samples for a training step, arrays over the cap sampled the
+    same way on every run."""
+    import numpy as np
+    import torch
+
+    b = _bench()
+    monkeypatch.setattr(b, "DUMP_MAX_ELEMS", 100)
+    monkeypatch.setattr(b, "DUMP_PARAM_SAMPLE", 50)
+    nets = (torch.nn.Linear(8, 8), torch.nn.Linear(4, 2))
+    outs = {"d_loss": torch.tensor(1.5), "out": torch.arange(300, dtype=torch.float64).reshape(3, 100)}
+    for run in ("a", "b"):
+        b.dump_outputs(str(tmp_path / run), outs, nets)
+    got = {p.stem: np.load(p) for p in (tmp_path / "a").iterdir()}
+    assert sorted(got) == ["d_loss", "discriminator_params", "generator_params", "out"]
+    assert all(v.dtype == np.float32 for v in got.values())
+    assert got["d_loss"].shape == () and float(got["d_loss"]) == 1.5
+    assert got["out"].shape == (100,) and len(set(got["out"].tolist())) == 100
+    assert got["generator_params"].shape == (50,) and got["discriminator_params"].shape == (10,)
+    for name, v in got.items():
+        assert np.array_equal(v, np.load(tmp_path / "b" / f"{name}.npy")), name
+
+
 def test_flop_model_matches_design():
     """DESIGN.md section 4: one step = B * [2 (F_G + 6 F_D) + K (3 F_G + 3 F_D)] with F_G = 521.4 GF, F_D = 35.7 GF."""
     b = _bench()

@@ -332,6 +332,28 @@ def test_unmodified_reference_wrapper_runs_on_these_modules(emu, generation_step
         del sys.modules[k]
 
 
+@pytest.mark.parametrize("generation_steps", [1, 2])
+def test_gan_step_matches_reference_wrapper_record(emu, generation_steps):
+    """training.gan_step on these modules logs the losses the reference's own DGMR.training_step logged on its own modules from the
+    same seeds (tests/golden/reference_wrapper_losses.json, written by make_golden.py): same construction, inputs, RNG draws and
+    optimiser settings; gan_step only leaves out the wrapper's discarded work, which changes none of the three losses."""
+    import json
+    import os
+
+    from parity_util import GOLDEN_DIR, module_gan_step
+
+    with open(os.path.join(GOLDEN_DIR, "reference_wrapper_losses.json")) as f:
+        rec = json.load(f)
+    cfg = rec["cfg"]
+    torch.manual_seed(rec["data_seed"])
+    x, y = torch.rand(2, 4, 1, 128, 128), torch.rand(2, 2, 1, 128, 128)
+    gen, disc = build_gan(dict(cfg, batch=2), seed=rec["init_seed"])
+    got = module_gan_step(gen, disc, x, y, seed=rec["step_seed"], device="cpu", generation_steps=generation_steps)["losses"]
+    for k, b in rec[f"generation_steps={generation_steps}"].items():
+        a = float(got[k.split("/")[1]])
+        assert abs(a - b) <= 2e-3 * max(abs(b), 1e-6), (k, a, b)
+
+
 @pytest.mark.parametrize("training", [True, False], ids=["train", "eval"])
 def test_upsample_gblock_subpixel_form(emu, training):
     """UpsampleGBlock with first_conv_3x3 in sub-pixel form (ops.upconv / ops._ConvBNRelu(up2): the four output phases as 2x2-tap
