@@ -291,6 +291,21 @@ int dgmr_grid_cell_bwd(const float* gen, const float* target, float cap, float c
 int dgmr_adam(float* p, const float* g, float* m, float* v, int64_t n, float lr, float beta1, float beta2,
               float eps, int step, float grad_scale, dgmr_stream_t stream);
 
+/* ---- ensemble statistics of K-member forecasts (Generator.sample; the ensemble the reference's unused DGMR(num_samples=6) describes,
+ * dgmr/dgmr.py:102), one pass over the ensemble.  P = T*C*H*W.
+ * ens [B][K][P] (the layout Generator.sample returns); target [B][P] or NULL; thr [n_thr] (device); mean [B][P];
+ * prob [n_thr][B][P] or NULL when n_thr == 0; crps [B][T*C][5] and ws (fp64, B*T*C*(H/16)*5 doubles) when target != NULL, else NULL
+ * (the target pointer is then never read).
+ *   mean[b][p]    = (sum of the members in member order) / K
+ *   prob[i][b][p] = count(ens[b][k][p] >= thr[i]) / K
+ *   crps[b][tc][s] = mean over the cells of frame (b, tc) at scale s of the ensemble CRPS
+ *                    (1/K) sum_k |x_k - y| - (1/(2K^2)) sum_{j,k} |x_j - x_k|,   sum_{j,k} |x_j - x_k| = 2 sum_i (2i - K + 1) x_(i)
+ *                    (x_(i) ascending, 0-based); scales s: 1 (pixels), 4x4 average, 4x4 maximum, 16x16 average, 16x16 maximum -- members and
+ *                    target pooled the same way over non-overlapping windows.
+ * 1 <= K <= 64, n_thr <= 8; with a target H and W must be multiples of 16.  No atomics: results are bitwise repeatable. */
+int dgmr_ensemble_stats(const float* ens, const float* target, const float* thr, int n_thr, float* mean, float* prob, float* crps, double* ws,
+                        int B, int K, int T, int C, int H, int W, dgmr_stream_t stream);
+
 /* y <- nearest TF32-representable value of x (cvt.rna.tf32.f32; y may alias x; idempotent); applied to activations before
  * they enter a tensor-core convolution: in place when the tensor feeds convolutions only, into a copy otherwise */
 int dgmr_round_tf32(const float* x, float* y, int64_t n, dgmr_stream_t stream);

@@ -384,6 +384,14 @@ class CudaBackend:
         self._call("dgmr_grid_cell_bwd", _f32(gen, "gen"), _f32(target, "target"), float(cap), float(coef), _f32(gout, "gout"),
                    _f32(dgen, "dgen"), gen.numel())
 
+    # -- ensemble statistics
+    def ensemble_stats(self, ens, target, thr, mean, prob, crps, ws, B, K, T, C, H, W):
+        n_thr = 0 if thr is None else thr.numel()
+        nb = 4.0 * B * T * C * H * W * (K + (target is not None) + 1 + n_thr)   # algorithmic bytes (profile only)
+        self._call("dgmr_ensemble_stats", _f32(ens, "ens"), _f32(target, "target"), _f32(thr, "thr"), n_thr, _f32(mean, "mean"),
+                   _f32(prob, "prob"), _f32(crps, "crps"), _f64(ws, "ws"), B, K, T, C, H, W, _flops=nb,
+                   _info=f"B{B} K{K} T{T} C{C} {H}x{W} thr{n_thr}{' +crps' if target is not None else ''} (GB/s)")
+
     def adam(self, p, g, m, v, lr, beta1, beta2, eps, step, grad_scale=1.0):
         self._call("dgmr_adam", _f32(p, "p"), _f32(g, "g"), _f32(m, "m"), _f32(v, "v"), p.numel(), float(lr), float(beta1),
                    float(beta2), float(eps), int(step), float(grad_scale))

@@ -269,15 +269,17 @@ class LatentConditioningStack(nn.Module, PyTorchModelHubMixin):
             self.att_block = AttentionLayer(output_channels // 4, output_channels // 4)
         self.l_block4 = LBlock(output_channels // 4, output_channels)
 
-    def sample_z(self, like: torch.Tensor) -> torch.Tensor:
+    def sample_z(self, like: torch.Tensor, k: int = 1) -> torch.Tensor:
+        """k successive draws (k reference calls' worth, in call order) as channels-last [k,1,H,W,C] on like's device."""
         s = tuple(self.shape) + (1,)
-        z = torch.normal(torch.zeros(s), torch.ones(s))  # == distribution.sample(self.shape), CPU RNG (:481)
+        zs = [torch.normal(torch.zeros(s), torch.ones(s)) for _ in range(k)]  # == distribution.sample(self.shape), CPU RNG (:481)
         # [C,H,W,1] -> channels-last [1,1,H,W,C]
-        z = z.squeeze(-1).permute(1, 2, 0).contiguous().unsqueeze(0).unsqueeze(0)
+        z = torch.stack(zs).squeeze(-1).permute(0, 2, 3, 1).contiguous().unsqueeze(1)
         return z.to(device=like.device, dtype=like.dtype)
 
-    def run(self, x: torch.Tensor):
-        z = self.sample_z(x)
+    def run(self, x: torch.Tensor, members: int = 1):
+        """-> channels-last [members,1,h,w,c]: one latent per ensemble member (batch 1 in the reference)."""
+        z = self.sample_z(x, members)
         z = self.conv_3x3.run(z, 1)
         z = self.l_block1.run(z)
         z = self.l_block2.run(z)

@@ -95,6 +95,10 @@ class DGMR(_Base, PyTorchModelHubMixin, library_name="DGMR",
     def forward(self, x):
         return self.generator(x)
 
+    def sample(self, x, num_samples=None):
+        """Eval-mode ensemble [B,K,T,C,H,W] of K = num_samples (default: the constructor's num_samples) forecasts: Generator.sample."""
+        return self.generator.sample(x, self.num_samples if num_samples is None else num_samples)
+
     # ------------------------------------------------------------------ reference schedule (dgmr/dgmr.py:137-218)
     def _disc_scores(self, images, future_images, predictions):
         generated_sequence = torch.cat([images, predictions], dim=1)

@@ -8,7 +8,7 @@ the reference's per-step calls.  Only the ConvGRU recurrence is sequential.
 """
 from __future__ import annotations
 
-from typing import List
+from typing import List, Optional
 
 import torch
 import torch.nn as nn
@@ -48,11 +48,36 @@ class Sampler(nn.Module, PyTorchModelHubMixin):
         self.conv_1x1 = SNConv(lc // 16, 4 * output_channels, (1, 1))
         self.output_channels = output_channels
 
-    def run(self, init_states: List[torch.Tensor], latent: torch.Tensor) -> torch.Tensor:
-        """init_states: channels-last [B,1,h,w,c], largest first; latent: channels-last [1,1,h,w,c].
-        Returns forecasts [B,T,C_out,H,W] (reference layout)."""
+    def max_image_elements(self, h: int, w: int) -> int:
+        """Elements of the largest per-image activation of one forecast step for an h x w latent grid: the widest tensor of every level
+        (gate pre-activations, blocks, and the up-block's first convolution at twice the resolution), for sizing batched launches."""
+        n = 0
+        for lvl, (gru, g, ug) in enumerate(((self.convGRU1, self.g1, self.up_g1), (self.convGRU2, self.g2, self.up_g2),
+                                            (self.convGRU3, self.g3, self.up_g3), (self.convGRU4, self.g4, self.up_g4))):
+            hw = (h << lvl) * (w << lvl)
+            cell = gru.cell
+            n = max(n, hw * max(cell.input_channels, 2 * cell.output_channels), hw * g.output_channels,
+                    4 * hw * max(ug.input_channels, ug.output_channels))
+        return n
+
+    def members_per_pass(self, batch: int, h: int, w: int) -> int:
+        """Largest member count M whose sampler pass (T*M*batch images per launch) keeps every tensor below 2^31 elements: the tensor-core
+        convolutions address with 32-bit offsets (N*H*W*Cout < 2^32, N*H*W < 2^31) and refuse larger launches."""
+        per_member = self.forecast_steps * batch * self.max_image_elements(h, w)
+        return max(1, ((1 << 31) - 1) // per_member)
+
+    def run(self, init_states: List[torch.Tensor], latent: torch.Tensor, out: Optional[torch.Tensor] = None, member0: int = 0) -> torch.Tensor:
+        """init_states: channels-last [B,1,h,w,c], largest first; latent: channels-last [M,1,h,w,c], one per ensemble member.
+        Returns forecasts [B,T,C_out,H,W] (reference layout) for M = 1, else [B,M,T,C_out,H,W].
+        The M members run as one batch of M*B images per step, ordered [T, M, B]; their conditioning states are the same.
+        out: write the members into out[:, member0:member0 + M] of an existing [B,K,T,C_out,H,W] tensor instead (no autograd)."""
         T = self.forecast_steps
         B = init_states[0].shape[0]
+        M = latent.shape[0]
+        if M > 1:
+            if self.training:
+                raise RuntimeError("Sampler.run: several members per pass are eval-mode only (train-mode statistics are per reference call)")
+            init_states = [ops.repeat_mid(s.reshape(1, s.numel()), M).reshape((M * B,) + tuple(s.shape[1:])) for s in init_states]
         levels = ((self.convGRU1, self.gru_conv_1x1, self.g1, self.up_g1),
                   (self.convGRU2, self.gru_conv_1x1_2, self.g2, self.up_g2),
                   (self.convGRU3, self.gru_conv_1x1_3, self.g3, self.up_g3),
@@ -65,7 +90,7 @@ class Sampler(nn.Module, PyTorchModelHubMixin):
         prefetch_sigmas(calls)
         hs = latent
         for lvl, (gru, c11, g, ug) in enumerate(levels):
-            # level 0: identical latent input at every step and for every sample (generators.py:146-149)
+            # level 0: identical latent input at every step and for every sample of a member (generators.py:146-149)
             # The level input is read by convolutions only: above level 0 it is the previous up-block's output, written tf32-rounded by that
             # block's last epilogue (conv_operand passes it through; unrounded tensors get one private rounded copy that both gate convs share).
             # The recurrence hands back the tf32-rounded copy of its outputs, which the 1x1 conv consumes as is.
@@ -75,14 +100,22 @@ class Sampler(nn.Module, PyTorchModelHubMixin):
             hs = g.run(hs, T)
             hs = ug.run(hs, T, round_out=(lvl < 3))      # levels 0-2: read by the next level's gate convolutions only
         hs = ops.mark_conv_only(self.bn.run(hs, T, relu=True, conv_only=True))
-        hs = self.conv_1x1.run(hs, T)  # [T*B,1,h,w,4*Co]
+        hs = self.conv_1x1.run(hs, T)  # [T*M*B,1,h,w,4*Co]
         _, _, h, w, c4 = hs.shape
         co = c4 // 4
+        F = co * 4 * h * w                                  # one output frame
+        K = M if out is None else out.shape[1]
         # PixelShuffle(2) + stack on dim 1 (:178,181) in one permute:
-        # out[b, t, co, 2h+i, 2w+j] = hs[t*B+b, h, w, co*4 + i*2 + j]
-        return ops.permute(hs, (B, T, co, 2 * h, 2 * w), (T, B, h, w, co, 2, 2),
-                           (B * h * w * c4, h * w * c4, w * c4, c4, 4, 2, 1),
-                           (co * 4 * h * w, T * co * 4 * h * w, 4 * w, 2, 4 * h * w, 2 * w, 1))
+        # out[b, member0 + m, t, co, 2h+i, 2w+j] = hs[(t*M + m)*B + b, h, w, co*4 + i*2 + j]
+        shape = [T, M, B, h, w, co, 2, 2]
+        sstr = [M * B * h * w * c4, B * h * w * c4, h * w * c4, w * c4, c4, 4, 2, 1]
+        dstr = [F, T * F, K * T * F, 4 * w, 2, 4 * h * w, 2 * w, 1]
+        if M == 1:                                          # no member axis: the reference's [B,T,...] permute
+            del shape[1], sstr[1], dstr[1]
+        if out is not None:
+            ops.permute_into(hs, out, shape, sstr, dstr, member0 * T * F)
+            return out
+        return ops.permute(hs, (B, T, co, 2 * h, 2 * w) if M == 1 else (B, M, T, co, 2 * h, 2 * w), shape, sstr, dstr)
 
     def forward(self, conditioning_states: List[torch.Tensor], latent_dim: torch.Tensor) -> torch.Tensor:
         """NCHW conditioning states (largest first) + latent [1,C,h,w] -> [B,T,C_out,H,W]."""
@@ -97,6 +130,36 @@ class Generator(nn.Module, PyTorchModelHubMixin):
         self.conditioning_stack = conditioning_stack
         self.latent_stack = latent_stack
         self.sampler = sampler
+
+    def sample(self, x: torch.Tensor, num_samples: int, members_per_pass: Optional[int] = None) -> torch.Tensor:
+        """An ensemble of `num_samples` eval-mode forecasts of the same context frames: x [B,T_in,C,H,W] -> [B,K,T,C_out,H,W].
+
+        Equals torch.stack([self(x) for _ in range(K)], dim=1) from the same CPU seed, drawing the K latents in the same order (the CPU RNG
+        ends in the same state), but runs the context stack once, the latent stack once at batch K and the sampler at M*B images per
+        launch for passes of M members.  M is the largest count whose tensors stay addressable by the tensor-core kernels
+        (Sampler.members_per_pass); `members_per_pass` can only lower it.  Eval mode only: in train mode every call advances the
+        spectral-norm vectors and BatchNorm statistics in call order."""
+        if self.training:
+            raise RuntimeError("Generator.sample is eval-mode only (call .eval() first)")
+        K = int(num_samples)
+        if K < 1:
+            raise RuntimeError(f"Generator.sample: num_samples must be >= 1, got {num_samples}")
+        if not all(hasattr(m, "run") for m in (self.conditioning_stack, self.latent_stack, self.sampler)):
+            raise RuntimeError("Generator.sample needs the package's own conditioning stacks and sampler")
+        B, H, W = x.shape[0], x.shape[-2], x.shape[-1]
+        lh, lw = self.latent_stack.shape[1], self.latent_stack.shape[2]
+        M = self.sampler.members_per_pass(B, lh, lw)
+        if members_per_pass is not None:
+            if members_per_pass < 1:
+                raise RuntimeError(f"Generator.sample: members_per_pass must be >= 1, got {members_per_pass}")
+            M = min(M, int(members_per_pass))
+        with torch.no_grad():
+            cond = list(self.conditioning_stack.run(x))     # no RNG and no batch statistics in eval mode: the same for every member
+            lat = self.latent_stack.run(x, K)               # [K,1,h,w,c]: the K draws in the sequential calls' order
+            out = torch.empty((B, K, self.sampler.forecast_steps, self.sampler.output_channels, H, W), device=x.device, dtype=torch.float32)
+            for k0 in range(0, K, M):
+                self.sampler.run(cond, lat[k0:k0 + M], out=out, member0=k0)
+        return out
 
     def forward(self, x: torch.Tensor):
         """x: [B,T_in,C,H,W] -> [B,T,C_out,H,W]; context stack, then latent stack, then sampler (RNG order)."""

@@ -11,6 +11,9 @@ device buffer before every replay, so seeded forecasts equal the eager path's.
 `train_mode=True` captures the TRAIN-mode forward without autograd instead -- what the discriminator phase of a GAN step runs twice
 (ref: dgmr/dgmr.py:159-160: `self(images)` under the generator's train mode, its gradients discarded): BatchNorm batch statistics, running
 statistics and the spectral-norm power iteration all advance on the device inside the replay, exactly as in the eager call.
+
+`num_samples=K > 1` captures the eval-mode ensemble forward `generator.sample(x, K)` instead -- every sampler pass of it in the one graph;
+each call draws the K latents in the reference's order into a static [K, ...] buffer and replays.
 """
 from __future__ import annotations
 
@@ -25,9 +28,16 @@ class GraphedGenerator:
     `x` must have the example's shape; the returned tensor is a static buffer that the next call overwrites (clone it to keep it).
     train_mode: capture the train-mode, no-grad forward (see the module docstring); the warm-up forwards needed before the capture would
     advance the module's buffers (spectral-norm u / v, BatchNorm running statistics), so they are saved and restored around it.
+    num_samples: K > 1 replays `generator.sample(x, K)` ([B,K,T,C,H,W], eval mode only).
     `launches`: C-ABI kernel launches recorded into the graph (what one replay executes without host calls)."""
 
-    def __init__(self, generator: torch.nn.Module, example_x: torch.Tensor, warmup: int = 2, train_mode: bool = False):
+    def __init__(self, generator: torch.nn.Module, example_x: torch.Tensor, warmup: int = 2, train_mode: bool = False,
+                 num_samples: int = 1):
+        self.num_samples = int(num_samples)
+        if self.num_samples < 1:
+            raise RuntimeError(f"GraphedGenerator: num_samples must be >= 1, got {num_samples}")
+        if train_mode and self.num_samples > 1:
+            raise RuntimeError("GraphedGenerator: num_samples > 1 is eval-mode only (train_mode=True replays single forwards)")
         if not example_x.is_cuda:
             raise RuntimeError("GraphedGenerator needs CUDA tensors (there is no CPU path)")
         be = _lib.backend()
@@ -41,7 +51,7 @@ class GraphedGenerator:
         self.generator = generator.train() if self.train_mode else generator.eval()
         self.x = example_x.detach().clone()
         self._latent = generator.latent_stack
-        self.z = self._latent.sample_z(self.x)           # static device buffer, refilled before every replay
+        self.z = self._latent.sample_z(self.x, self.num_samples)   # static device buffer, refilled before every replay
         saved = [(b, b.detach().clone()) for b in generator.buffers()] if self.train_mode else []
         side = torch.cuda.Stream()
         side.wait_stream(torch.cuda.current_stream())
@@ -67,10 +77,10 @@ class GraphedGenerator:
 
     def _forward_static(self):
         orig = self._latent.sample_z
-        self._latent.sample_z = lambda like: self.z       # the graph reads the static buffer; the draw itself happens outside
+        self._latent.sample_z = lambda like, k=1: self.z  # the graph reads the static buffer; the draw itself happens outside
         try:
             with torch.no_grad():
-                return self.generator(self.x)
+                return self.generator(self.x) if self.num_samples == 1 else self.generator.sample(self.x, self.num_samples)
         finally:
             self._latent.sample_z = orig
 
@@ -79,7 +89,7 @@ class GraphedGenerator:
             raise RuntimeError(f"GraphedGenerator was captured for input shape {tuple(self.x.shape)}, got {tuple(x.shape)}")
         if self.generator.training != self.train_mode:
             raise RuntimeError("GraphedGenerator: the generator's train / eval mode changed since the capture")
-        z = self._latent.sample_z(self.x)                 # CPU draw in the reference's RNG order + host->device copy
+        z = self._latent.sample_z(self.x, self.num_samples)   # CPU draws in the reference's RNG order + host->device copy
         self.z.copy_(z, non_blocking=True)
         self.x.copy_(x, non_blocking=True)
         self.graph.replay()

@@ -34,9 +34,9 @@ class ConvGRUCell(nn.Module):
     # ---- channels-last multi-step engine -------------------------------------------------
     def run_sequence(self, xs: torch.Tensor, h0: torch.Tensor, T: int, shared_input: bool = False,
                      rounded_out: bool = False) -> torch.Tensor:
-        """xs: [T*B,1,H,W,Cx] timestep-major (or [1,1,H,W,Cx] with shared_input=True: the same input at every
-        step and for every batch element, as at the sampler's first level, ref: generators.py:146-149);
-        h0: [B,1,H,W,Ch].  Returns [T*B,1,H,W,Ch].  rounded_out: the caller feeds the result to convolutions only and
+        """xs: [T*B,1,H,W,Cx] timestep-major (or [M,1,H,W,Cx] with shared_input=True: the same input at every step, one per
+        member m for the B/M consecutive batch elements of that member, as at the sampler's first level, ref: generators.py:146-149,
+        where M = 1); h0: [B,1,H,W,Ch].  Returns [T*B,1,H,W,Ch].  rounded_out: the caller feeds the result to convolutions only and
         accepts the tf32-rounded copy the recurrence writes anyway (fused path on the tensor cores)."""
         ch = self.output_channels
         cx = self.input_channels - ch
@@ -65,13 +65,16 @@ class ConvGRUCell(nn.Module):
 
     @staticmethod
     def _x_part(xs, w, bias, sc, T, B, cx, shared_input):
-        """Input-dependent part of a gate pre-activation for all T steps: [T, B, 1, H, W, Cout] (bias and sigma_t applied)."""
+        """Input-dependent part of a gate pre-activation for all T steps: [T, B, 1, H, W, Cout] (bias and sigma_t applied).
+        shared_input: xs [M,1,H,W,Cx] holds one input per member; the convolution runs on the T*M distinct images and its result is
+        broadcast over each member's B/M batch elements."""
         if shared_input:
+            m = xs.shape[0]
             p = xs.numel()
-            x_rep = ops.mark_conv_only(ops.repeat_mid(xs.reshape(1, p), T).reshape((T,) + tuple(xs.shape[1:])))
-            xp = ops.conv(x_rep, w, bias, sc, None, 0, cx, T, ACT_NONE)  # [T,1,H,W,Cout]
-            q = xp.numel() // T
-            return ops.repeat_mid(xp.reshape(T, q), B).reshape((T, B) + tuple(xp.shape[1:]))
+            x_rep = ops.mark_conv_only(ops.repeat_mid(xs.reshape(1, p), T).reshape((T * m,) + tuple(xs.shape[1:])))
+            xp = ops.conv(x_rep, w, bias, sc, None, 0, cx, T, ACT_NONE)  # [T*M,1,H,W,Cout]
+            q = xp.numel() // (T * m)
+            return ops.repeat_mid(xp.reshape(T * m, q), B // m).reshape((T, B) + tuple(xp.shape[1:]))
         xp = ops.conv(xs, w, bias, sc, None, 0, cx, T, ACT_NONE)
         return xp.reshape((T, B) + tuple(xp.shape[1:]))
 

@@ -108,6 +108,11 @@ def permute(src, out_shape, shape, sstr, dstr, src_off=0, dst_off=0):
     return _Permute.apply(src, tuple(out_shape), tuple(shape), tuple(sstr), tuple(dstr), src_off, dst_off)
 
 
+def permute_into(src, dst, shape, sstr, dstr, dst_off=0):
+    """`permute` without autograd into an existing tensor at element offset dst_off (inference outputs assembled in place)."""
+    _be().permute(_c(src), dst, tuple(shape), tuple(sstr), tuple(dstr), False, 0, dst_off)
+
+
 def nchw_to_cl(x: torch.Tensor) -> torch.Tensor:
     """[N,C,H,W] or [N,C,D,H,W] -> [N,D,H,W,C]."""
     if x.dim() == 4:
